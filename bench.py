@@ -199,6 +199,40 @@ def feat_formula(ids, dim, device):
     return v.to(torch.float32) * (1.0 / 1048576.0)
 
 
+DUMP_BYTES = 60 << 20  # --dump-outputs: all arrays together, under 64 MB (10^6 bytes) with the .npy headers
+
+
+def last_step_outputs(n_id, adjs, x):
+    """What the timed call returned in its last step, as host arrays: ids and sizes as float64 (exact below 2^53), the
+    gathered rows as float32."""
+    out = {"n_id": n_id.cpu().double().numpy()}
+    for i, a in enumerate(adjs):
+        out[f"adj{i}_edge_index"] = a.edge_index.cpu().double().numpy()
+        out[f"adj{i}_size"] = torch.as_tensor(a.size).double().numpy()
+    out["x"] = x.cpu().float().numpy()
+    return out
+
+
+def dump_outputs(path, arrays, budget=DUMP_BYTES, seed=0):
+    """Write every array as path/<name>.npy, smallest first, each within an even share of what is left of `budget`.  An
+    array larger than its share is replaced by a sample along its longest axis, drawn by a generator with a fixed seed;
+    <name>_index.npy (float64) holds the sampled positions, so that two runs with the same arguments write the same files."""
+    import numpy as np
+    os.makedirs(path, exist_ok=True)
+    left = budget
+    for i, (name, a) in enumerate(sorted(arrays.items(), key=lambda t: t[1].nbytes)):
+        share = left // (len(arrays) - i)
+        if a.nbytes > share:
+            axis = int(np.argmax(a.shape))
+            m = share // (a.nbytes // a.shape[axis] + 8)
+            pick = np.sort(np.random.default_rng(seed).choice(a.shape[axis], m, replace=False))
+            np.save(os.path.join(path, f"{name}_index.npy"), pick.astype(np.float64))
+            a = np.take(a, pick, axis=axis)
+            left -= pick.nbytes
+        np.save(os.path.join(path, f"{name}.npy"), a)
+        left -= a.nbytes
+
+
 class ClockSampler(threading.Thread):
     """nvidia-smi clocks / throttle reasons while the timed region runs (B200_PROFILING.md)."""
     FIELDS = "clocks.sm,clocks.max.sm,clocks_event_reasons.hw_slowdown,clocks_event_reasons.hw_thermal_slowdown," \
@@ -691,6 +725,8 @@ def run_ours(args, cfg, rank, world, local_rank):
         barrier()
         rep_ms.append((a0.elapsed_time(a1), edges_r))
         launches = _lib.launch_count() - launches0
+    # the last step's results are copied to the host here, between timed regions, and written at the end of the run
+    last_outputs = last_step_outputs(n_id, adjs, res) if args.dump_outputs and rank == 0 else None
     rep_rates = sorted(e / (ms * 1e-3) for ms, e in rep_ms)
     # the reported K-step region is the median repeat (by rate)
     med = sorted(rep_ms, key=lambda t: t[1] / t[0])[len(rep_ms) // 2]
@@ -904,10 +940,13 @@ def run_ours(args, cfg, rank, world, local_rank):
             except Exception as e:  # the reference calls exit(1) on CUDA errors; anything catchable is reported
                 out["ref_gpu_baseline"] = {"unavailable": f"{type(e).__name__}: {e}"}
         out["cpu_baseline"] = cpu_baseline_sample(cfg, indptr_cpu, indices_cpu, timed_host)
+    if last_outputs is not None:
+        dump_outputs(args.dump_outputs, last_outputs)
     return out
 
 
 def main():
+    sys.dont_write_bytecode = True  # the benchmark writes nothing into the source tree, which may be read-only
     ap = argparse.ArgumentParser()
     ap.add_argument("--gpus", type=int, default=1)
     ap.add_argument("--steps", type=int, default=20)
@@ -932,7 +971,12 @@ def main():
                     help="`value` from sample() + feature[n_id] as two calls instead of sample_and_gather")
     ap.add_argument("--overlap", action="store_true",
                     help="run the sampler on its own high-priority stream so sample(i+1) overlaps gather(i)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write what the timed call returned in its last step as DIR/<name>.npy (float32 / float64, at "
+                         "most 64 MB in all; a seeded sample of larger outputs), to compare two builds on the same inputs")
     args = ap.parse_args()
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     cfg = dict(CONFIGS[args.config])
     if args.feat_dim:
         cfg["feat_dim"] = args.feat_dim

@@ -98,3 +98,24 @@ def test_host_table_folds_large_tables():
     assert rows == 100 and x.shape == (100, 8)
     x, rows = bench.host_table(50, 8)
     assert rows == 50
+
+
+def test_dump_outputs_fit_the_budget_and_repeat(tmp_path):
+    rng = np.random.default_rng(0)
+    arrays = {"n_id": np.arange(1000, dtype=np.float64), "adj0_edge_index": rng.integers(0, 1000, (2, 30000)).astype(np.float64),
+              "x": rng.random((20000, 16), dtype=np.float32)}
+    budget = 600_000
+    for run in ("a", "b"):
+        bench.dump_outputs(str(tmp_path / run), arrays, budget=budget)
+    files = sorted(p.name for p in (tmp_path / "a").iterdir())
+    assert files == ["adj0_edge_index.npy", "adj0_edge_index_index.npy", "n_id.npy", "x.npy", "x_index.npy"]
+    assert sum(p.stat().st_size for p in (tmp_path / "a").iterdir()) <= budget + 5 * 128  # + the .npy headers
+    for f in files:
+        a, b = np.load(tmp_path / "a" / f), np.load(tmp_path / "b" / f)
+        assert a.dtype in (np.float32, np.float64) and np.array_equal(a, b)  # same arguments, same files
+    load = lambda f: np.load(tmp_path / "a" / f)  # noqa: E731
+    assert np.array_equal(load("n_id.npy"), arrays["n_id"])  # within its share: whole
+    pick = load("x_index.npy").astype(np.int64)
+    assert np.array_equal(load("x.npy"), arrays["x"][pick]) and len(np.unique(pick)) == len(pick)
+    pick = load("adj0_edge_index_index.npy").astype(np.int64)
+    assert np.array_equal(load("adj0_edge_index.npy"), arrays["adj0_edge_index"][:, pick])

@@ -3,7 +3,8 @@
   * XORWOW restatement  == NVIDIA curand_kernel.h run on the host            (tests/golden/xorwow_kat.json)
   * counts / verbatim rows / reindex == the reference CPU extension           (tests/golden/ref_cpu_kat.json)
   * structural validity == the reference's only sampler assertion             (tests/cpp/test_quiver_cpu.cpp:32-75)
-When oracle/_ref/ holds the live builds (this container), the same checks also run against them directly.
+When oracle/_ref/ holds the live builds, the same checks also run against them directly; without them,
+test_live_reference_cpu_extension checks the outputs of that build stored in tests/golden/ref_cpu_ext_kat.json.
 """
 import json
 import os
@@ -12,6 +13,7 @@ import numpy as np
 import pytest
 
 from graphs import MINI, powerlaw_csr, simple_graph
+from reference_outputs import ReferenceOutputs
 
 
 def _golden_graph(name, meta):
@@ -117,22 +119,28 @@ def test_sampler_is_uniform(oracle):
     assert chi2 < 80.0  # 39 dof: p(chi2 > 80) ~ 1e-4
 
 
-def test_live_reference_cpu_extension(oracle):
-    ref = oracle.load_reference()
-    if ref is None:
-        pytest.skip("oracle/_ref/torch_quiver_ref not built on this machine")
+def test_live_reference_cpu_extension(oracle, golden_dir):
+    live = oracle.load_reference()
+    ref = ReferenceOutputs(os.path.join(golden_dir, "ref_cpu_ext_kat.json"), live,
+                           "the reference's CPU extension compiled unmodified (oracle/build_ref.py)", deterministic=False)
     import torch
     indptr, indices = powerlaw_csr(2000, 20.0, seed=9)
-    cq = ref.cpu_quiver_from_csr_array(torch.from_numpy(indptr), torch.from_numpy(indices))
+    cq = live.cpu_quiver_from_csr_array(torch.from_numpy(indptr), torch.from_numpy(indices)) if live else None
     seeds = np.random.default_rng(1).permutation(2000)[:256]
     for k in (3, 10, 2000):
-        out, cnt = cq.sample_neighbor(torch.from_numpy(seeds), k)
+        reindexed = None
+        if live is not None:
+            out, cnt = cq.sample_neighbor(torch.from_numpy(seeds), k)
+            f, r, c = cq.reindex_single(torch.from_numpy(seeds), out, cnt)
+            reindexed = {"frontier": f, "row_idx": r, "col_idx": c}
+        drawn = ref.arrays(f"k={k}", {"out": out, "cnt": cnt} if live is not None else None)
+        out, cnt = drawn["out"], drawn["cnt"]
         counts, _, tot = oracle.sample_counts(indptr, seeds, k)
-        assert cnt.tolist() == counts.tolist() and out.numel() == tot
-        assert oracle.validate_sample(indptr, indices, seeds, k, counts, out.numpy()) == 0
-        f, r, c = cq.reindex_single(torch.from_numpy(seeds), out, cnt)
-        of, orow, ocol = oracle.reindex(seeds, out.numpy(), counts)
-        assert f.tolist() == of.tolist() and r.tolist() == orow.tolist() and c.tolist() == ocol.tolist()
+        assert cnt.tolist() == counts.tolist() and out.size == tot
+        assert oracle.validate_sample(indptr, indices, seeds, k, counts, out) == 0
+        of, orow, ocol = oracle.reindex(seeds, out, counts)
+        ref.check(f"k={k}/reindex_single", {"frontier": of, "row_idx": orow, "col_idx": ocol}, reindexed)
+    ref.save()
 
 
 def test_gather_oracle_is_tensor_indexing(oracle):
